@@ -21,6 +21,10 @@ barrier and the max-over-ranks time.
              timed region), against MEASURED_PEAKS.json's sustained bf16 figure (fp16 runs at the same rate).
   cpu_baseline  the oracle port (oracle/w2l_oracle.py, torch CPU fp32 = the reference's own arithmetic) on
              the host cores, N=128 4-D batch (inference.py's default batch), rank 0 at N=1 only.
+
+--dump-outputs DIR writes what rank 0's last timed step returned as DIR/<name>.npy (float32): generator_out.npy,
+the (B,3,T,96,96) prediction, or losses.npy for --workload train.  Inputs and weights depend only on the arguments,
+so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -32,10 +36,29 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it
 
 FLOP_PER_CROP = 2 * 3966984192  # SURVEY.md §8(d): 3 966.98 MMAC per 96x96 crop
 METRIC = "96x96 face-crops/sec (B=128, T=5, mel 80x16)"
 B_DEFAULT, T_DEFAULT = 128, 5
+DUMP_BYTES = 64 * 10**6  # --dump-outputs: all arrays together
+
+
+def dump_outputs(path, arrays):
+    """Write each tensor of `arrays` as <path>/<name>.npy in float32.  One that does not fit what is left of DUMP_BYTES
+    is cut to a fixed seeded sample of its leading-axis rows (kept in order), the same rows on every run."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES - 4096 * len(arrays)  # room for the .npy headers
+    for name, t in arrays.items():
+        t = t.detach().float().cpu()
+        if t.numel() * 4 > left:
+            rows = left // (t[0].numel() * 4)
+            pick = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values
+            t = t[pick]
+        left -= t.numel() * 4
+        np.save(os.path.join(path, name + ".npy"), t.numpy())
 
 
 def load_peaks():
@@ -264,7 +287,7 @@ def measure_extra(dev):
     return out
 
 
-def measure_train(dev, rank, world, steps, warmup, B=64, T=5, syncnet_wt=0.03, profile_out=None):
+def measure_train(dev, rank, world, steps, warmup, B=64, T=5, syncnet_wt=0.03, profile_out=None, dump_dir=None):
     """BASELINE configs[4]: one wav2lip_train.py:210-231 iteration per step (generator train-mode forward, get_sync_loss
     through the frozen expert, L1, backward, gradient all-reduce over NCCL when world > 1, Adam), bf16 operands, B=64
     windows x T=5 frames per GPU, everything native (w2l_wav2lip_train_step).  Inputs resident on the device; CUDA-event
@@ -308,12 +331,15 @@ def measure_train(dev, rank, world, steps, warmup, B=64, T=5, syncnet_wt=0.03, p
     e1.record(stream)
     torch.cuda.synchronize(dev)
     barrier()
+    last_losses = losses.cpu()   # the step reuses its loss buffer: copy the last timed step's before anything else runs
     ms = max_over_ranks(e0.elapsed_time(e1), dev) / steps
     launches = (ctx.launch_count() - l0) // steps
     gen_f = ctx.lib.w2l_train_flops(ctx.h, _lib.NET_GENERATOR)
     syn_f = ctx.lib.w2l_train_flops(ctx.h, _lib.NET_SYNCNET)
     flop = 3.0 * gen_f + 2.0 * syn_f       # forward + dgrad + wgrad of the generator; forward + dgrad of the frozen expert
-    lv = [float(v) for v in losses.cpu()]
+    lv = [float(v) for v in last_losses]
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"losses": last_losses})
     n_param = sum(p.numel() for p in model.parameters())
     if profile_out and rank == 0:
         rows = ctx.train_profile(_lib.NET_GENERATOR, iters=3, stream=stream.cuda_stream) + \
@@ -346,7 +372,7 @@ def run_reference(args, rank, world):
     with torch.no_grad():
         for _ in range(max(1, min(args.warmup, 1))):
             O.generator_forward(sd, mel, face)
-        steps = max(1, min(args.steps, 3))   # ~14 s per step on the box's host: the whole arm stays under ~2 minutes
+        steps = args.steps   # a step takes seconds on the host cores: pass a small --steps for this arm
         t0 = time.perf_counter()
         for _ in range(steps):
             O.generator_forward(sd, mel, face)
@@ -383,7 +409,11 @@ def main():
                     help="weak (default, the driver's mode): --batch windows PER GPU.  strong: --batch is the GLOBAL batch, split over the ranks")
     ap.add_argument("--workload", default="infer", choices=["infer", "train"],
                     help="infer: the headline metric (default).  train: BASELINE configs[4], one training iteration per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -413,7 +443,8 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     if args.workload == "train":
         tb = 64 if args.batch == B_DEFAULT else args.batch
-        r = measure_train(dev, rank, world, args.steps, args.warmup, B=tb, T=args.frames, profile_out=args.profile_out)
+        r = measure_train(dev, rank, world, args.steps, args.warmup, B=tb, T=args.frames, profile_out=args.profile_out,
+                          dump_dir=args.dump_outputs)
         if rank == 0:
             line = {"metric": "wav2lip_train.py iterations: 96x96 face-crops/sec trained (B=64/GPU, T=5, bf16)", "value": r["crops_per_s"],
                     "unit": "crops/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"],
@@ -477,6 +508,7 @@ def main():
         e1.record(stream)
         torch.cuda.synchronize(dev)
         t_wall1 = time.time()
+        last_out = out
         barrier()
         launches = ctx.launch_count() - l0
         ms = e0.elapsed_time(e1)
@@ -588,6 +620,9 @@ def main():
         cpu = {"value": v, "unit": "crops/s", "cores": cores, "kind": "port",
                "sample": f"one N=128 4-D batch (inference.py batch) = {dt:.2f} s of oracle/w2l_oracle.py (torch CPU fp32; "
                          f"{cores} threads = the fastest of 8/16/32/64/{os.cpu_count()} on this host)"}
+
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"generator_out": last_out})
 
     if rank == 0:
         line = {

@@ -156,8 +156,39 @@ def main():
         out["wav_checksum_" + kind] = np.float64(np.abs(wav.astype(np.float64)).sum())
     out["mel_basis"] = M.mel_basis()
     np.savez_compressed(os.path.join(HERE, "mel.npz"), **out)
-    for f in ("generator", "syncnet", "disc", "mel"):
+    reference_seed3()
+    for f in ("generator", "syncnet", "disc", "mel", "reference_seed3"):
         print(f, os.path.getsize(os.path.join(HERE, f + ".npz")) // 1024, "KiB")
+
+
+def reference_seed3():
+    """Full outputs of the three reference networks on a second weight seed (3) and input seed (5), for
+    tests/test_oracle_golden.py::test_oracle_vs_live_reference."""
+    out = {}
+    sd = O.make_state_dict("generator", 3)
+    m = Wav2Lip()
+    m.load_state_dict(sd, strict=True)
+    m.eval()
+    mel, face = O.make_generator_inputs(1, 5)
+    with torch.no_grad():
+        out["gen_out"] = m(mel, face).numpy()
+    out["gen_sd_checksum"] = np.float64(checksum_sd(sd))
+    out["gen_in_checksum"] = np.array([mel.double().abs().sum().item(), face.double().abs().sum().item()])
+    sd = O.make_state_dict("syncnet", 3)
+    s = SyncNet_color()
+    s.load_state_dict(sd, strict=True)
+    s.eval()
+    mel, face = O.make_syncnet_inputs(2, 5)
+    with torch.no_grad():
+        a, v = s(mel, face)
+    out["sync_a"], out["sync_v"] = a.numpy(), v.numpy()
+    sd = O.make_state_dict("disc", 3)
+    d = Wav2Lip_disc_qual()
+    d.load_state_dict(sd, strict=True)
+    d.eval()
+    with torch.no_grad():
+        out["disc_out"] = d(O.make_disc_inputs(1, 5, 5)).numpy()
+    np.savez_compressed(os.path.join(HERE, "reference_seed3.npz"), **out)
 
 
 if __name__ == "__main__":

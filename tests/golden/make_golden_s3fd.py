@@ -64,6 +64,19 @@ def main():
     out["big_shapes"] = np.array([list(o.shape) for o in o2], dtype=np.int32)
     np.savez_compressed(os.path.join(HERE, "s3fd.npz"), **out)
     print("wrote s3fd.npz:", cand.shape, [len(k) for k in keeps], [tuple(o.shape) for o in olist])
+    seed3(ref)
+
+
+def seed3(ref):
+    """The 12 output maps at a second weight seed (3) on a 70x90 frame (seed 5), for
+    tests/test_s3fd_oracle.py::test_oracle_against_live_reference."""
+    net = ref["net_s3fd"].s3fd()
+    net.load_state_dict(S.make_state_dict(3), strict=True)
+    net.eval()
+    with torch.no_grad():
+        olist = net(S.preprocess(S.make_images(1, 70, 90, seed=5)))
+    np.savez_compressed(os.path.join(HERE, "s3fd_seed3.npz"), **{f"o{i}": o.numpy() for i, o in enumerate(olist)})
+    print("wrote s3fd_seed3.npz:", [tuple(o.shape) for o in olist])
 
 
 if __name__ == "__main__":

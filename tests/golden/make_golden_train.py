@@ -50,7 +50,7 @@ def train_inputs(B, seed):
 
 def main():
     torch.manual_seed(0)
-    torch.set_num_threads(os.cpu_count() or 1)
+    torch.set_num_threads(8)   # the fp32 sums depend on the thread count: tests/test_train_oracle.py runs with 8 too
     out = {}
     B = 2
 

@@ -1,11 +1,8 @@
 """The oracle restatement (oracle/w2l_oracle.py) against the committed outputs of the REAL
-reference modules (tests/golden/*.npz, made by tests/golden/make_golden.py), and — when the
-reference checkout is present (build container) — against the live reference."""
+reference modules (tests/golden/*.npz, made by tests/golden/make_golden.py)."""
 import os
-import sys
 
 import numpy as np
-import pytest
 import torch
 
 from oracle import w2l_oracle as O
@@ -92,27 +89,25 @@ def test_disc_oracle_matches_reference_golden(golden_dir):
         _check_fp(name, _fp(taps[name]), g["disc_fp/" + name])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference checkout not present")
-def test_oracle_vs_live_reference():
-    sys.path.insert(0, "/root/reference")
-    try:
-        from models import Wav2Lip, SyncNet_color, Wav2Lip_disc_qual
-    finally:
-        sys.path.remove("/root/reference")
+def test_oracle_vs_live_reference(golden_dir):
+    """A second weight and input seed against the full outputs of the reference modules
+    (tests/golden/reference_seed3.npz, made by make_golden.py)."""
+    g = np.load(os.path.join(golden_dir, "reference_seed3.npz"))
     sd = O.make_state_dict("generator", 3)
-    m = Wav2Lip(); m.load_state_dict(sd, strict=True); m.eval()
+    chk = sum(v.double().abs().sum().item() for v in sd.values() if v.dtype.is_floating_point)
+    assert abs(chk - float(g["gen_sd_checksum"])) <= 1e-9 * chk, "seeded weights drifted (torch RNG changed?)"
     mel, face = O.make_generator_inputs(1, 5)
+    np.testing.assert_allclose([mel.double().abs().sum().item(), face.double().abs().sum().item()],
+                               g["gen_in_checksum"], rtol=1e-12)
     with torch.no_grad():
-        np.testing.assert_allclose(O.generator_forward(sd, mel, face).numpy(), m(mel, face).numpy(), atol=TOL)
+        np.testing.assert_allclose(O.generator_forward(sd, mel, face).numpy(), g["gen_out"], atol=TOL)
     sd = O.make_state_dict("syncnet", 3)
-    s = SyncNet_color(); s.load_state_dict(sd, strict=True); s.eval()
     mel, face = O.make_syncnet_inputs(2, 5)
     with torch.no_grad():
-        a0, v0 = s(mel, face); a1, v1 = O.syncnet_forward(sd, mel, face)
-    np.testing.assert_allclose(a1.numpy(), a0.numpy(), atol=TOL)
-    np.testing.assert_allclose(v1.numpy(), v0.numpy(), atol=TOL)
+        a1, v1 = O.syncnet_forward(sd, mel, face)
+    np.testing.assert_allclose(a1.numpy(), g["sync_a"], atol=TOL)
+    np.testing.assert_allclose(v1.numpy(), g["sync_v"], atol=TOL)
     sd = O.make_state_dict("disc", 3)
-    d = Wav2Lip_disc_qual(); d.load_state_dict(sd, strict=True); d.eval()
     fr = O.make_disc_inputs(1, 5, 5)
     with torch.no_grad():
-        np.testing.assert_allclose(O.disc_forward(sd, fr).numpy(), d(fr).numpy(), atol=TOL)
+        np.testing.assert_allclose(O.disc_forward(sd, fr).numpy(), g["disc_out"], atol=TOL)

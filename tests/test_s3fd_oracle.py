@@ -1,9 +1,8 @@
 """Scope row f4 (S3FD face detector), CPU part: the restatement oracle/s3fd_oracle.py against vectors produced by the REAL
-reference modules (tests/golden/s3fd.npz <- tests/golden/make_golden_s3fd.py), against the live reference when it is present,
-and the product's host-side post-processing (wav2lip_b200/face_detection/detection/sfd/sfd_detector.py: vectorised NumPy)
-against the reference's own candidate array and NMS keep lists."""
+reference modules (tests/golden/s3fd.npz, s3fd_seed3.npz <- tests/golden/make_golden_s3fd.py), and the product's
+host-side post-processing (wav2lip_b200/face_detection/detection/sfd/sfd_detector.py: vectorised NumPy) against the
+reference's own candidate array and NMS keep lists."""
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -68,18 +67,16 @@ def test_mirror_state_dict_is_the_references():
         m(torch.zeros(1, 3, 64, 64))          # CPU tensor: no fallback
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/face_detection"), reason="reference tree not present")
-def test_oracle_against_live_reference():
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    import make_golden_s3fd as G
-    ref = G.load_reference()
+def test_oracle_against_live_reference(golden_dir):
+    """A second weight seed and frame size against the reference module's 12 output maps
+    (tests/golden/s3fd_seed3.npz, made by make_golden_s3fd.py)."""
+    g = np.load(os.path.join(golden_dir, "s3fd_seed3.npz"))
     sd = S.make_state_dict(3)
-    net = ref["net_s3fd"].s3fd()
-    net.load_state_dict(sd, strict=True)
-    net.eval()
     imgs = S.make_images(1, 70, 90, seed=5)
     with torch.no_grad():
-        a = net(S.preprocess(imgs))
         b = S.forward(sd, S.preprocess(imgs))
-    for x, y in zip(a, b):
-        assert torch.allclose(x, y, rtol=1e-4, atol=1e-5)
+    assert len(b) == 12
+    for i, y in enumerate(b):
+        x = torch.from_numpy(g[f"o{i}"])
+        assert x.shape == y.shape, i
+        assert torch.allclose(x, y, rtol=1e-4, atol=1e-5), i
